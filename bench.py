@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W                (our arm: CUDA path through the C ABI)
   python bench.py --impl reference --gpus N --steps K --warmup W   (reference arm: CPU restatement, host cores)
+  python bench.py ... --dump-outputs DIR                        (also writes what the last timed step computed, DIR/<name>.npy)
 
 Workload (config.workload): BASELINE.json configs[1] -- 300 frames, 384x224, 16x12 bilinear depth-scale
 grid, hierarchical2 frame pairs, matchSeparation 10 (reference default), Cauchy 0.5, PerFrame intrinsics,
@@ -76,6 +77,27 @@ def initial_state(sc, cfg, stride):
     x = sc.gt_state(stride, 7, nd)
     rng = np.random.default_rng(7)
     return x + rng.normal(0, 0.005, x.shape)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes float64 arrays as out_dir/<name>.npy so that two builds can be compared output for output.  Arrays of one row per
+    frame that would exceed DUMP_LIMIT_BYTES together keep a fixed, seeded sample of frames; sampled_frames.npy lists them."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    per_frame = [k for k, v in arrays.items() if v.ndim == 2]
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES and per_frame:
+        n = arrays[per_frame[0]].shape[0]
+        row_bytes = sum(arrays[k][0].nbytes for k in per_frame) + 8      # + the entry of sampled_frames
+        keep = (DUMP_LIMIT_BYTES - 4096 - (total - n * (row_bytes - 8))) // row_bytes   # 4 KiB for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: (v[rows] if k in per_frame else v) for k, v in arrays.items()}
+        arrays["sampled_frames"] = rows.astype(np.float64)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def shard_pairs(pairs, offs, rec, rank, nranks):
@@ -235,6 +257,7 @@ def run_ours(args):
     wall = time.perf_counter() - t0
     launches = P.launch_count() - l0
     clocks = sampler.stop()
+    outputs = P.iteration_outputs() if args.dump_outputs else None      # before the calls below overwrite the device buffers
     ms = tm["iter_ms"]
     if world > 1:
         tt = torch.tensor([ms], dtype=torch.float64, device="cuda")
@@ -299,6 +322,8 @@ def run_ours(args):
         for _ in range(args.e2e_steps):
             s, xs = call(); its += s.iterations
         sync_all(); dt = time.perf_counter() - t1
+        if outputs is not None:
+            outputs.update(e2e_state=xs, e2e_costs=np.array([s.initial_cost, s.final_cost]))
         h2d = float(lr.nbytes + lp.nbytes + lo.nbytes + x0.nbytes + med.nbytes + cfg.num_frames)
         if world > 1:
             tt = torch.tensor([dt, -h2d], dtype=torch.float64, device="cuda")
@@ -313,6 +338,8 @@ def run_ours(args):
             dist.barrier()
             dist.destroy_process_group()
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -392,7 +419,12 @@ def main():
     ap.add_argument("--legacy-update", action="store_true", help="A/B: round-1 cp.async update GEMM instead of the TMA-fed persistent kernel")
     ap.add_argument("--side-ipc", type=int, default=0, help="A/B: items-per-CTA cap of the overlapped (side-stream) update launches")
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (gradient, LM step, candidate state, costs; and the last e2e call's final "
+                         "state and costs) as DIR/<name>.npy, float64, at most 64 MB in all")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

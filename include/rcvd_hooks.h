@@ -24,6 +24,10 @@ int32_t rcvd_debug_linear_solve(rcvd_problem* p, const double* S, const double* 
  * assembled H), |S g|, cost, |g|_2, |y|_2, non-positive-pivot flag}: the parity evidence bench.py prints at the size it times */
 int32_t rcvd_debug_linear_residual(rcvd_problem* p, double radius, double out[6]);
 
+/* what the last step of rcvd_time_iteration computed, in the caller's frame order (N x stride doubles each): the gradient at the
+ * state, the LM step and the candidate state (state + step, projected onto the bounds); costs = {cost at the state, candidate cost} */
+int32_t rcvd_debug_iteration_outputs(rcvd_problem* p, double* gradient, double* step, double* candidate, double costs[2]);
+
 /* per-kernel-class device time of one factorisation + solve: out_ms[0..5] = load, potrf, trinv, trsm, update GEMM,
  * substitution; [6] = update-GEMM launches, [7] = their algorithmic flops.  reps > 0: serialised on one stream;
  * reps < 0: two-stream overlap kept, main-stream view. */

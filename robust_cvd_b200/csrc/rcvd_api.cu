@@ -1448,6 +1448,16 @@ RCVD_API int32_t rcvd_time_iteration(rcvd_problem* p, int32_t iters, double radi
   *ms_iter = tt / iters; if (ms_acc) *ms_acc = ta / iters; if (ms_lin) *ms_lin = tl / iters; if (ms_cost) *ms_cost = tc / iters;
   return RCVD_OK;
 }
+// Bench hook: the arrays the last step of rcvd_time_iteration left on the device, in the caller's frame order (N x stride each).
+RCVD_API int32_t rcvd_debug_iteration_outputs(rcvd_problem* p, double* gradient, double* step, double* candidate, double costs[2]) {
+  if (!p || !gradient || !step || !candidate || !costs) return set_err(RCVD_ERR_INVALID, "null argument");
+  if (!p->structure_ready) return set_err(RCVD_ERR_INVALID, "no iteration has run on this problem");
+  SET_DEVICE(p->device);
+  costs[0] = p->h_scal[SC_COST]; costs[1] = p->h_scal[SC_CAND];
+  int rc = download_frames(p, gradient, p->d_g, p->L.nf, p->L.npad, p->L.nf); if (rc) return rc;
+  if ((rc = download_frames(p, step, p->d_delta, p->L.nf, p->L.npad, p->L.nf))) return rc;
+  return download_frames(p, candidate, p->d_xc, p->L.nf, p->L.nf, p->L.nf);
+}
 // Bench hook: one factorisation + solve, un-captured on a single stream with one CUDA event per launch; returns the
 // summed device time per kernel class: out_ms[0..5] = load, potrf, trinv, trsm, update GEMM (k_gemm_nt), substitution;
 // out_ms[6] = number of k_gemm_nt update launches, out_ms[7] = algorithmic flops of those GEMMs.

@@ -152,6 +152,14 @@ class Problem:
         _check(self.L.rcvd_time_iteration(self.h, C.c_int32(iters), C.c_double(radius), C.byref(a), C.byref(b), C.byref(c), C.byref(d)))
         return {"iter_ms": a.value, "accumulate_ms": b.value, "linear_ms": c.value, "cost_ms": d.value}
 
+    def iteration_outputs(self):
+        """Bench hook: gradient, LM step and candidate state ([N, stride] each) and {cost, candidate cost} of the last
+        time_iteration step."""
+        g, step, xc = (np.empty((self.N, self.stride), np.float64) for _ in range(3))
+        costs = np.empty(2, np.float64)
+        _check(self.L.rcvd_debug_iteration_outputs(self.h, _p(g, C.c_double), _p(step, C.c_double), _p(xc, C.c_double), _p(costs, C.c_double)))
+        return {"gradient": g, "step": step, "candidate_state": xc, "costs": costs}
+
     def structure_info(self):
         out = (C.c_int32 * 8)()
         _check(self.L.rcvd_structure_info(self.h, out))

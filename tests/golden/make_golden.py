@@ -1,6 +1,6 @@
-"""Generates the committed golden fixtures.  Run in the build container (needs /root/reference for the
-pure-Python pieces of the reference; the solver goldens come from the CPU oracle because the reference's
-C++ path cannot be built here -- see DESIGN.md "Oracle")."""
+"""Generates the committed golden fixtures: `python tests/golden/make_golden.py <robust_cvd checkout>` (the reference's
+pure-Python pieces are imported from that checkout; the solver goldens come from the CPU oracle because the reference's
+C++ path cannot be built without its dependencies -- see DESIGN.md "Oracle")."""
 import json
 import os
 import sys
@@ -10,10 +10,11 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+REFERENCE = None          # path of a robust_cvd checkout (command line)
 
 
 def golden_pairs():
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REFERENCE)
     from utils import frame_sampling as fs
     from utils.frame_range import FrameRange, OptionalSet
     out = {}
@@ -47,16 +48,16 @@ def golden_solver():
 def golden_raw_images():
     """.raw wire format: files written by the reference's own utils/image_io.py::save_raw_float32_image (imported unchanged)."""
     import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_image_io", "/root/reference/utils/image_io.py")
+    spec = importlib.util.spec_from_file_location("ref_image_io", os.path.join(REFERENCE, "utils", "image_io.py"))
     io = importlib.util.module_from_spec(spec)
     try:
         spec.loader.exec_module(io)
     except Exception:      # the module imports cv2 / other helpers at the top; only the two raw functions are needed
-        src = open("/root/reference/utils/image_io.py").read()
+        src = open(os.path.join(REFERENCE, "utils", "image_io.py")).read()
         a = src.index("def load_raw_float32_image"); b = src.index("def save_raw_float32_image")
         end = src.find("\ndef ", b + 10)
         ns = {"np": np, "struct": __import__("struct")}
-        exec(compile(src[a:end if end > 0 else len(src)], "/root/reference/utils/image_io.py", "exec"), ns)      # executed in place, not copied
+        exec(compile(src[a:end if end > 0 else len(src)], os.path.join(REFERENCE, "utils", "image_io.py"), "exec"), ns)      # executed in place, not copied
         io = type("io", (), {k: staticmethod(v) for k, v in ns.items() if callable(v)})
     rng = np.random.default_rng(4)
     disp = (rng.random((5, 7)) * 2 + 0.1).astype(np.float32); disp[1, 2] = 0.0; disp[3, 3] = np.inf
@@ -96,7 +97,7 @@ def golden_geometry():
     The fine-tuning loss consumes the poses the C++ optimiser produced with this model, so StaticSceneCost's geometry
     (sign conventions, NDC mapping, aspect handling, focal definition) must reproduce it: tests/test_oracle.py checks that the
     oracle's residuals vanish on these correspondences."""
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REFERENCE)
     import torch
     from utils import geometry as G
     from robust_cvd_b200.synthetic import rodrigues
@@ -121,10 +122,111 @@ def golden_geometry():
     np.savez_compressed(os.path.join(HERE, "ref_python_geometry.npz"), **out)
 
 
+def golden_pose_optimization_trace():
+    """Every lib_python attribute read, call and assignment that the reference's own pose_optimization.py (imported unchanged)
+    makes in PoseOptimizer(...) and optimize_poses() on the 8-frame scene of tests/test_host.py, with what each returned, recorded
+    on a machine without a GPU: optimize_poses() ends with the call that refuses to run without one.  Objects are numbered in
+    order of appearance (0 = the module), paths inside the scene directory are written relative to "{root}".
+    tests/test_host.py replays the sequence against lib_python."""
+    import importlib
+    import shutil
+    import tempfile
+    sys.path.insert(0, os.path.join(ROOT, "robust_cvd_b200", "host"))
+    import lib_python
+    from tests.test_host import write_scene8
+    root = tempfile.mkdtemp(prefix="rcvd_trace_")
+    write_scene8(root)
+    trace = {"init": [], "optimize_poses": []}
+    phase = ["init"]
+    primitive = (bool, int, float, str, type(None))
+
+    def enc(v):
+        if isinstance(v, Recorder):
+            return {"ref": object.__getattribute__(v, "_id")}
+        if isinstance(v, (list, tuple)):
+            return [enc(x) for x in v]
+        assert isinstance(v, primitive), type(v)
+        return v.replace(root, "{root}") if isinstance(v, str) else v
+
+    def raw(v):
+        if isinstance(v, Recorder):
+            return object.__getattribute__(v, "_obj")
+        return [raw(x) for x in v] if isinstance(v, list) else v
+
+    def result(op, v):
+        trace[phase[0]].append(op)
+        if isinstance(v, primitive) or (isinstance(v, (list, tuple)) and all(isinstance(x, primitive) for x in v)):
+            op["out"] = enc(v)
+            return v
+        r = Recorder(v)
+        op["out"] = enc(r)
+        return r
+
+    class Recorder:
+        count = [0]
+
+        def __init__(self, obj):
+            object.__setattr__(self, "_obj", obj)
+            object.__setattr__(self, "_id", Recorder.count[0])
+            Recorder.count[0] += 1
+
+        def __getattr__(self, name):
+            v = getattr(object.__getattribute__(self, "_obj"), name)
+            if name.startswith("__"):          # import machinery
+                return v
+            return result({"op": "get", "obj": object.__getattribute__(self, "_id"), "name": name}, v)
+
+        def __setattr__(self, name, value):
+            trace[phase[0]].append({"op": "set", "obj": object.__getattribute__(self, "_id"), "name": name, "value": enc(value)})
+            setattr(object.__getattribute__(self, "_obj"), name, raw(value))
+
+        def __call__(self, *args, **kwargs):
+            assert not kwargs
+            op = {"op": "call", "obj": object.__getattribute__(self, "_id"), "args": enc(list(args))}
+            try:
+                v = object.__getattribute__(self, "_obj")(*[raw(a) for a in args])
+            except Exception as e:
+                op["raises"] = {"type": type(e).__name__, "message": str(e)}
+                trace[phase[0]].append(op)
+                raise
+            return result(op, v)
+
+    dflt = lib_python.DepthVideoPoseOptimizer.Params()
+    sys.modules["lib_python"] = Recorder(lib_python)
+    sys.path.insert(0, REFERENCE)
+    try:
+        po = importlib.import_module("pose_optimization")
+        from utils.helpers import Nestedspace
+        o = Nestedspace()
+        for k, v in dict(max_iterations=50, num_threads=12, num_steps=4, robustness=0.5, static_loss_type="ReproDisparity", static_spatial_weight=1.0,
+                         static_depth_weight=1.0, smooth_loss_type="ReproDisparityLaplacian", smooth_static_weight=0.0, smooth_dynamic_weight=0.0,
+                         position_regularization=0.0, scale_regularization=1.0, scale_regularization_grid_size=10, deformation_regularization_initial=1.0,
+                         deformation_regularization_final=0.1, adaptive_deformation_cost=0.0, spatial_deformation_regularization=1.0,
+                         graduate_deformation_regularization=False, focal_regularization=1.0, coarse_to_fine=True, ctf_long=dflt.ctfLong, ctf_short=dflt.ctfShort,
+                         deferred_spatial_opt=False, dso_long=4, dso_short=3, focal_long=dflt.focalLong, intr_opt="PerFrame", fix_poses=False,
+                         fix_depth_transforms=False, fix_spatial_transforms=False, use_global_scale=False, dynamic_constraints="Mask").items():
+            setattr(o, k, v)
+        os.environ["RCVD_CONSTRAINT_BUILDER"] = "host"          # as in tests/test_host.py
+        opt = po.PoseOptimizer(root, "midas2", list(range(8)), o)
+        phase[0] = "optimize_poses"
+        try:
+            opt.optimize_poses()
+            raise AssertionError("optimize_poses() ran: record the trace on a machine without a GPU")
+        except RuntimeError:
+            pass
+    finally:
+        sys.modules["lib_python"] = lib_python
+        shutil.rmtree(root, ignore_errors=True)
+    with open(os.path.join(HERE, "ref_pose_optimization_trace.json"), "w") as f:       # one operation per line
+        f.write("{\n" + ",\n".join(f'"{k}": [\n' + ",\n".join(json.dumps(op) for op in ops) + "\n]" for k, ops in trace.items()) + "\n}\n")
+
+
 if __name__ == "__main__":
+    REFERENCE = sys.argv[1]
     golden_geometry()
     golden_pairs()
     golden_solver()
     golden_raw_images()
     golden_host_restatements()
+    golden_pose_optimization_trace()
     print("golden fixtures written")

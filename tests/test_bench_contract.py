@@ -1,11 +1,13 @@
-"""bench.py on the CPU: the workloads follow BASELINE.json's configs, the pair sharding is a partition, and the reference arm
-(`--impl reference`, the CPU restatement on the host cores) prints a line with every key of the measurement contract."""
+"""bench.py: the workloads follow BASELINE.json's configs, the pair sharding is a partition, the reference arm (`--impl reference`,
+the CPU restatement on the host cores) prints a line with every key of the measurement contract, and `--dump-outputs` writes what
+the timed path computed (on the GPU)."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -46,6 +48,41 @@ def test_pair_sharding_is_a_balanced_partition():
         assert lo[-1] == lr.shape[0]
     assert sorted(seen) == sorted(tuple(p) for p in pairs) and sum(counts) == rec.shape[0]
     assert max(counts) - min(counts) <= np.diff(offs).max()
+
+
+def test_dump_outputs_keeps_a_fixed_sample_under_the_limit(tmp_path, monkeypatch):
+    import bench
+    rng = np.random.default_rng(1)
+    arrays = {"a": rng.normal(size=(100, 30)), "b": rng.normal(size=(100, 30)).astype(np.float32), "costs": np.array([2.0, 1.0])}
+    bench.dump_outputs(str(tmp_path / "full"), arrays)
+    assert sorted(os.listdir(tmp_path / "full")) == ["a.npy", "b.npy", "costs.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "full" / "a.npy"), arrays["a"])
+    assert np.load(tmp_path / "full" / "b.npy").dtype == np.float64
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4096 + 20 * (2 * 30 * 8 + 8) + 16)       # room for 20 of the 100 frames
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    got = {f: np.load(tmp_path / "s1" / f) for f in os.listdir(tmp_path / "s1")}
+    rows = got["sampled_frames.npy"].astype(int)
+    assert len(rows) == 20 and np.all(np.diff(rows) > 0) and rows[-1] < 100
+    np.testing.assert_array_equal(got["a.npy"], arrays["a"][rows]); np.testing.assert_array_equal(got["costs.npy"], arrays["costs"])
+    assert sum(v.nbytes for v in got.values()) <= bench.DUMP_LIMIT_BYTES
+    np.testing.assert_array_equal(np.load(tmp_path / "s2" / "sampled_frames.npy"), got["sampled_frames.npy"])
+
+
+@pytest.mark.gpu
+def test_bench_dumps_what_the_timed_steps_computed(tmp_path):
+    """`--steps` sets the number of timed steps and `--dump-outputs` writes the arrays of the last one and of the last e2e call."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "config1_8f_128x96_grid4x4_sep10", "--steps", "4", "--warmup", "1",
+                          "--skip-cpu", "--skip-pose-opt", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads(out.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 4
+    got = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sorted(got) == ["candidate_state", "costs", "e2e_costs", "e2e_state", "gradient", "step"]
+    stride = d["config"]["structure"]["stride"]
+    for k in ("candidate_state", "e2e_state", "gradient", "step"):
+        assert got[k].shape == (8, stride) and got[k].dtype == np.float64 and np.isfinite(got[k]).all(), k
+    assert 0 < got["e2e_costs"][1] < got["e2e_costs"][0] and abs(got["costs"][0] - got["e2e_costs"][0]) <= 1e-11 * got["costs"][0]
 
 
 def test_reference_arm_prints_the_contract_line():

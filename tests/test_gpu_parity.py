@@ -59,6 +59,24 @@ def test_linear_solve(name, overrides):
         assert np.linalg.norm(y2 - y) / np.linalg.norm(y) < 1e-9
 
 
+def test_iteration_outputs_are_one_lm_step():
+    """Problem.iteration_outputs (what bench.py --dump-outputs writes) after time_iteration: cost and gradient at the state, the
+    Jacobi-scaled LM step of trust radius 1e4 on the oracle's normal matrix, and the cost at the candidate state."""
+    sc, cfg, O, G, x = _both(helpers.VARIANTS[0][1])
+    G.time_iteration(iters=2, radius=1e4)
+    out = G.iteration_outputs()
+    co, go = O.evaluate(True)
+    assert abs(out["costs"][0] - co) <= 1e-11 * abs(co), (out["costs"], co)
+    assert np.abs(out["gradient"].ravel() - go).max() <= 1e-9 * max(1.0, np.abs(go).max())
+    H = O.normal_matrix_dense()
+    S = 1.0 / (1.0 + np.sqrt(np.diag(H)))
+    D2 = np.clip(S * S * np.diag(H), 1e-6, 1e32) / 1e4
+    step = -S * np.linalg.solve(H * S[:, None] * S[None, :] + np.diag(D2), S * go)
+    assert np.linalg.norm(out["step"].ravel() - step) <= 1e-6 * np.linalg.norm(step)
+    G.set_state(out["candidate_state"])
+    assert abs(G.evaluate() - out["costs"][1]) <= 1e-11 * abs(out["costs"][1])
+
+
 @pytest.mark.parametrize("name,overrides", helpers.VARIANTS, ids=[v[0] for v in helpers.VARIANTS])
 def test_lm_solve_matches_oracle(name, overrides):
     sc, cfg, O, G, x = _both(overrides)

@@ -2,6 +2,7 @@
 restatement, problem assembly arrays, pose conversions, coarse-to-fine split -- everything of the
 drop-in boundary that does not need the GPU."""
 import os
+import re
 import shutil
 import struct
 import sys
@@ -26,9 +27,7 @@ def _host_constraint_builder(monkeypatch):
     monkeypatch.setenv("RCVD_CONSTRAINT_BUILDER", "host")
 
 
-@pytest.fixture(scope="module")
-def scene_dir(tmp_path_factory):
-    root = str(tmp_path_factory.mktemp("scene8"))
+def write_scene8(root):
     sc = synthetic.Scene(8, 128, 96, seed=3)
     rng = np.random.default_rng(5)
     masks = []
@@ -36,6 +35,11 @@ def scene_dir(tmp_path_factory):
         m = np.full((96, 128), 255, np.uint8); cx, cy = rng.integers(30, 100), rng.integers(30, 70); m[cy - 8:cy + 8, cx - 10:cx + 10] = 0; masks.append(m)
     pairs = synthetic_files.write_scene(sc, root, dynamic_masks=masks)
     return sc, root, pairs, masks
+
+
+@pytest.fixture(scope="module")
+def scene_dir(tmp_path_factory):
+    return write_scene8(str(tmp_path_factory.mktemp("scene8")))
 
 
 def _open(root):
@@ -356,35 +360,49 @@ def test_grid_split_resamples_bilinearly(scene_dir):
     assert abs(f.intrinsics.hFov - 2 * np.arctan(np.float32(0.3461538376301239))) < 1e-6
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/pose_optimization.py"), reason="reference checkout only exists in the build container")
-def test_reference_pose_optimization_py_runs_unchanged_up_to_the_solve(scene_dir):
-    """The reference's own pose_optimization.py, unmodified, against our lib_python: everything up to the
-    device solve runs here; the solve itself must refuse to run without a GPU (no CPU fallback)."""
-    import importlib, types
-    sc, root, pairs, masks = scene_dir
-    for f in ("flow_constraints.dat",):
-        if os.path.exists(f"{root}/{f}"): os.remove(f"{root}/{f}")
-    sys.path.insert(0, "/root/reference")
-    try:
-        po = importlib.import_module("pose_optimization")
-        from utils.helpers import Nestedspace
-        dflt = lp.DepthVideoPoseOptimizer.Params()
-        o = Nestedspace()
-        for k, v in dict(max_iterations=50, num_threads=12, num_steps=4, robustness=0.5, static_loss_type="ReproDisparity", static_spatial_weight=1.0,
-                         static_depth_weight=1.0, smooth_loss_type="ReproDisparityLaplacian", smooth_static_weight=0.0, smooth_dynamic_weight=0.0,
-                         position_regularization=0.0, scale_regularization=1.0, scale_regularization_grid_size=10, deformation_regularization_initial=1.0,
-                         deformation_regularization_final=0.1, adaptive_deformation_cost=0.0, spatial_deformation_regularization=1.0,
-                         graduate_deformation_regularization=False, focal_regularization=1.0, coarse_to_fine=True, ctf_long=dflt.ctfLong, ctf_short=dflt.ctfShort,
-                         deferred_spatial_opt=False, dso_long=4, dso_short=3, focal_long=dflt.focalLong, intr_opt="PerFrame", fix_poses=False,
-                         fix_depth_transforms=False, fix_spatial_transforms=False, use_global_scale=False, dynamic_constraints="Mask").items():
-            setattr(o, k, v)
-        opt = po.PoseOptimizer(root, "midas2", list(range(8)), o)
-        assert os.path.exists(f"{root}/flow_constraints.dat") and os.path.exists(f"{root}/video.dat")
-        import torch
-        if not torch.cuda.is_available():
-            with pytest.raises(RuntimeError, match="no CPU fallback|no usable CUDA device"):
-                opt.optimize_poses()
-    finally:
-        sys.path.remove("/root/reference")
-        for m in [k for k in sys.modules if k == "pose_optimization" or k.startswith("utils")]:
-            sys.modules.pop(m, None)
+NO_CPU_FALLBACK = "no CPU fallback|no usable CUDA device"
+
+
+def _replay(ops, objs, root):
+    """Replays a recorded lib_python call sequence (tests/golden/make_golden.py records it): every attribute read, call and
+    assignment, each primitive result checked against the recorded one.  A recorded failure may only end the sequence and must be
+    the refusal to run without a GPU; returns whether the sequence ended in it."""
+    def dec(v):
+        if isinstance(v, dict):
+            return objs[v["ref"]]
+        if isinstance(v, list):
+            return [dec(x) for x in v]
+        return v.replace("{root}", root) if isinstance(v, str) else v
+    for i, op in enumerate(ops):
+        o = objs[op["obj"]]
+        if op["op"] == "set":
+            setattr(o, op["name"], dec(op["value"]))
+            continue
+        if "raises" in op:
+            assert i == len(ops) - 1 and op["raises"]["type"] == "RuntimeError" and re.search(NO_CPU_FALLBACK, op["raises"]["message"]), op
+            with pytest.raises(RuntimeError, match=NO_CPU_FALLBACK):
+                o(*dec(op["args"]))
+            return True
+        out = getattr(o, op["name"]) if op["op"] == "get" else o(*dec(op["args"]))
+        if isinstance(op["out"], dict):
+            objs[op["out"]["ref"]] = out
+        else:
+            assert (list(out) if isinstance(out, tuple) else out) == dec(op["out"]), (i, op)
+    return False
+
+
+def test_reference_pose_optimization_py_runs_unchanged_up_to_the_solve(tmp_path):
+    """The calls the reference's own pose_optimization.py makes into lib_python (PoseOptimizer(...) and optimize_poses() on
+    this module's 8-frame scene, recorded from the unmodified script into tests/golden/ref_pose_optimization_trace.json) run
+    against our lib_python with the same results: everything up to the device solve runs here; the solve itself must refuse to
+    run without a GPU (no CPU fallback)."""
+    import json
+    trace = json.load(open(os.path.join(GOLDEN, "ref_pose_optimization_trace.json")))
+    root = str(tmp_path / "scene8")
+    write_scene8(root)
+    objs = {0: lp}
+    assert not _replay(trace["init"], objs, root)
+    assert os.path.exists(f"{root}/flow_constraints.dat") and os.path.exists(f"{root}/video.dat")
+    import torch
+    if not torch.cuda.is_available():
+        assert _replay(trace["optimize_poses"], objs, root)
