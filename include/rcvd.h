@@ -255,6 +255,35 @@ int32_t rcvd_flow_guided_filter(const rcvd_filter_params* prm, int32_t device, c
                                 const float* fwd_flow, const uint8_t* fwd_mask, const float* bwd_flow, const uint8_t* bwd_mask,
                                 const int32_t* far_pairs, const float* far_flow, const uint8_t* far_mask, float* out);
 
+/* ---- bilateral depth filter ----
+ * Replaces DepthVideoProcessor::bilateralFilter (lib/Processor.cpp:183-313).  Arrays are indexed by a local frame index
+ * 0..num_frames-1 over a consecutive block of the video that holds every temporal window, i.e. from
+ * max(0, first - frame_radius) to min(numFrames - 1, last + frame_radius); frames no window reaches may hold anything.
+ *   depth        [num_frames][height][width] f32     transformed depth of depth stream 0 (DepthFrame::depth())
+ *   color        [num_frames][height][width][3] f32  "down" colour stream (CV_32FC3); only read, and may be NULL, when color_sigma <= 0
+ *   out_frames   [num_out] strictly ascending local indices of the frames to filter (Params::frameRange)
+ *   xform_cfg    depth transform of stream 0 and xform_params [num_out][depth params] of each output frame: only read with
+ *                in_place and frame_radius > 0
+ *   out          [num_out][height][width] f32
+ * in_place (depthStream == 0): the reference writes each filtered frame back to stream 0 before the next one, so a later
+ * window reads the depth transform applied to the filtered image; frames are then filtered one launch at a time in order.
+ * Float32 arithmetic in the reference's operation order; weights use the accurate expf (1 ulp from libm's).  A median pixel
+ * whose cumulative weight never reaches half the total (NaN weights) is 0, where the reference leaves it uninitialised.
+ * spatial_radius is limited by the TMA box (256 elements) and the shared memory of one CTA: at most 24 with the colour term,
+ * about 70 without; a larger radius returns RCVD_ERR_INVALID. */
+typedef struct rcvd_bilateral_params {
+  int32_t num_frames, num_out;
+  int32_t width, height;
+  int32_t spatial_radius; /* Params::spatialRadius (lib/Processor.h:66) */
+  int32_t frame_radius;   /* Params::frameRadius */
+  int32_t median;         /* Params::median: 0 weighted mean, 1 weighted median */
+  int32_t in_place;       /* 1: outputs replace the filtered frames' depth before later windows read them (depthStream == 0) */
+  float depth_sigma;      /* Params::depthSigma; <= 0 switches the depth term off */
+  float color_sigma;      /* Params::colorSigma; <= 0 switches the colour term off */
+} rcvd_bilateral_params;
+int32_t rcvd_bilateral_filter(const rcvd_bilateral_params* prm, int32_t device, const float* depth, const float* color,
+                              const int32_t* out_frames, const rcvd_config* xform_cfg, const double* xform_params, float* out);
+
 /* ---- GPU flow-constraint builder (SURVEY.md section 8f-2) ----
  * Replaces FlowConstraintsCollection::compute (lib/FlowConstraints.cpp:401-550: admission tests, cv::cornerMinEigenVal
  * priorities) and sampleConstraints (:352-397: greedy disc sampler) for a batch of frame pairs and frame triplets.

@@ -7,7 +7,8 @@
 extern "C" {
 #endif
 
-/* kernels launched so far by this handle / by the filter / by the constraint builder (the "did the CUDA path run" evidence) */
+/* kernels launched so far by this handle / by the flow-guided and bilateral filters / by the constraint builder (the "did the
+ * CUDA path run" evidence) */
 int64_t rcvd_launch_count(rcvd_problem* p);
 int64_t rcvd_filter_launch_count(void);
 int64_t rcvd_builder_launch_count(void);

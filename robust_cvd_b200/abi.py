@@ -74,6 +74,12 @@ class FilterParams(C.Structure):
                                          "frame_radius", "spatial_radius", "median", "num_far")] + [("inv_aspect", C.c_float)]
 
 
+class BilateralParams(C.Structure):
+    """rcvd_bilateral_params (include/rcvd.h)."""
+    _fields_ = [(n, C.c_int32) for n in ("num_frames", "num_out", "width", "height", "spatial_radius", "frame_radius", "median", "in_place")] + \
+               [("depth_sigma", C.c_float), ("color_sigma", C.c_float)]
+
+
 class BuilderParams(C.Structure):
     """rcvd_builder_params (include/rcvd.h)."""
     _fields_ = [(n, C.c_int32) for n in ("num_frames", "width", "height", "dyn_width", "dyn_height", "match_separation", "num_pairs", "num_triplets")] + \

@@ -23,6 +23,7 @@
 #include "rcvd_update.cuh"
 #include "rcvd_dense.cuh"
 #include "rcvd_filter.cuh"
+#include "rcvd_bilateral.cuh"
 #include "rcvd_builder.cuh"
 static int64_t g_filter_launches = 0;
 
@@ -1793,6 +1794,141 @@ RCVD_API int32_t rcvd_flow_guided_filter(const rcvd_filter_params* prm, int32_t 
   return rc;
 }
 RCVD_API int64_t rcvd_filter_launch_count() { return g_filter_launches; }
+
+// ---------------------------------------------------------------------------
+// Bilateral depth filter (rcvd_bilateral.cuh)
+// ---------------------------------------------------------------------------
+// 3-D float32 tensor map {d0, d1, d2} with byte strides s1 (dimension 1) and s2 (dimension 2), box {b0, b1, 1}, zero fill outside
+static bool encode_f32_3d(CUtensorMap* m, void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1, uint64_t s2, uint32_t b0, uint32_t b1) {
+  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
+                               CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  static EncodeFn fn = nullptr;
+  if (!fn) {
+    void* p = nullptr; cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || !p || q != cudaDriverEntryPointSuccess) { cudaGetLastError(); return false; }
+    fn = (EncodeFn)p;
+  }
+  const cuuint64_t gdim[3] = {d0, d1, d2}, gstr[2] = {s1, s2};
+  const cuuint32_t box[3] = {b0, b1, 1u}, estr[3] = {1u, 1u, 1u};
+  return fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+template <bool MEDIAN, bool IN_PLACE>
+static cudaError_t bilateral_prepare(size_t smem) { return cudaFuncSetAttribute(k_bilateral<MEDIAN, IN_PLACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); }
+template <bool MEDIAN, bool IN_PLACE>
+static void bilateral_launch(dim3 grid, size_t smem, cudaStream_t st, const CUtensorMap& td, const CUtensorMap& tc, const BilateralArgs& a) {
+  k_bilateral<MEDIAN, IN_PLACE><<<grid, kBilThreads, smem, st>>>(td, tc, a);
+}
+
+RCVD_API int32_t rcvd_bilateral_filter(const rcvd_bilateral_params* prm, int32_t device, const float* depth, const float* color, const int32_t* out_frames,
+                                       const rcvd_config* xform_cfg, const double* xform_params, float* out) {
+  if (!prm || !depth || !out_frames || !out) return set_err(RCVD_ERR_INVALID, "null argument");
+  const rcvd_bilateral_params& q = *prm;
+  if (q.num_frames <= 0 || q.num_out <= 0 || q.width <= 0 || q.height <= 0 || q.spatial_radius < 0 || q.frame_radius < 0)
+    return set_err(RCVD_ERR_INVALID, "bad bilateral filter parameters");
+  for (int k = 0; k < q.num_out; ++k)
+    if (out_frames[k] < 0 || out_frames[k] >= q.num_frames || (k > 0 && out_frames[k] <= out_frames[k - 1]))
+      return set_err(RCVD_ERR_INVALID, "output frames must be ascending local frame indices below num_frames");
+  const bool use_c = q.color_sigma > 0.f;
+  if (use_c && !color) return set_err(RCVD_ERR_INVALID, "colour frames missing (colorSigma > 0)");
+  const bool in_place = q.in_place && q.frame_radius > 0;   // with frameRadius 0 no window reaches a filtered frame
+  Layout L{};
+  if (in_place && (!xform_cfg || !xform_params || !make_layout(*xform_cfg, L))) return set_err(RCVD_ERR_INVALID, "in-place filtering needs a supported depth transform and its parameters");
+  const int r = q.spatial_radius, w = q.width, h = q.height, F = q.num_frames;
+  // padded planes (rcvd_bilateral.cuh): halo boxes start at (tile_y, tile_x) of the padded plane; every extent <= 256 elements
+  const int pad_l = (r + 3) / 4 * 4, box_w = kBilTW + 2 * pad_l, box_h = kBilTH + 2 * r, cbox_w = 3 * box_w;
+  const uint32_t depth_bytes = (uint32_t)((box_w * box_h * 4 + 1023) / 1024 * 1024);
+  const uint32_t stage_bytes = depth_bytes + (use_c ? (uint32_t)((cbox_w * box_h * 4 + 1023) / 1024 * 1024) : 0u);
+  const size_t smem = 2 * (size_t)stage_bytes + 2 * sizeof(uint64_t);
+  int ndev = 0;
+  cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess || ndev <= 0 || device < 0 || device >= ndev)
+    return set_err(RCVD_ERR_NO_DEVICE, "no usable CUDA device (%s); this library has no CPU fallback", e != cudaSuccess ? cudaGetErrorString(e) : "device ordinal out of range");
+  SET_DEVICE(device);
+  int smem_max = 0; CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+  if (box_w > 256 || box_h > 256 || (use_c && cbox_w > 256) || smem > (size_t)smem_max)
+    return set_err(RCVD_ERR_INVALID, "spatialRadius %d is too large: the %d x %d halo tile of one frame%s does not fit the TMA box / shared-memory limits", r,
+                   box_w, box_h, use_c ? " with colour" : "");
+  const int Wp = std::max((pad_l + w + r + 3) / 4 * 4, box_w), Hp = std::max(h + 2 * r, box_h);
+  const size_t dplane = (size_t)Wp * Hp, cplane = 3 * dplane;
+  const int P = F + (in_place ? q.num_out : 0);
+  const int window = (int)std::min<int64_t>(2 * (int64_t)q.frame_radius + 1, F);
+  const int max_samples = (2 * r + 1) * (2 * r + 1) * window;
+  // the weighted median sorts a per-pixel sample row: the scratch is bounded to ~1 GiB by filtering frame chunks, and row bands of a
+  // frame when one frame alone is larger
+  const size_t row_scratch = (size_t)w * max_samples * sizeof(float2), limit = (size_t)1 << 30;
+  int zmax = in_place ? 1 : std::min(q.num_out, 65535), band = h;
+  if (q.median) {
+    if (row_scratch * h <= limit) zmax = (int)std::min<size_t>((size_t)zmax, limit / (row_scratch * h));
+    else { zmax = 1; band = (int)std::max<size_t>(1, limit / row_scratch); if (band >= kBilTH) band -= band % kBilTH; }
+  }
+  std::vector<int> retrans(F, -1);
+  for (int k = 0; k < q.num_out; ++k) retrans[out_frames[k]] = k;
+  std::vector<double> xp;
+  if (in_place) {
+    xp.assign((size_t)q.num_out * L.nf, 0.0);
+    for (int k = 0; k < q.num_out; ++k) for (int i = 0; i < L.nd; ++i) xp[(size_t)k * L.nf + L.offD + i] = xform_params[(size_t)k * L.nd + i];
+  }
+  cudaStream_t st; CK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+  std::vector<void*> bufs; bool ok = true;
+  auto dev = [&](size_t bytes) -> void* { void* ptr = nullptr; if (cudaMallocAsync(&ptr, std::max<size_t>(bytes, 16), st) != cudaSuccess) { ok = false; cudaGetLastError(); return nullptr; } bufs.push_back(ptr); return ptr; };
+  auto up = [&](const void* src, size_t bytes) -> void* { void* d = dev(bytes); if (d && bytes) cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, st); return d; };
+  BilateralArgs a{};
+  a.depth = (float*)dev((size_t)P * dplane * 4);
+  if (a.depth) {
+    cudaMemsetAsync(a.depth, 0, (size_t)P * dplane * 4, st);
+    for (int f = 0; f < F; ++f)
+      cudaMemcpy2DAsync(a.depth + f * dplane + (size_t)r * Wp + pad_l, (size_t)Wp * 4, depth + (size_t)f * h * w, (size_t)w * 4, (size_t)w * 4, h, cudaMemcpyHostToDevice, st);
+  }
+  if (use_c) {
+    float* c = (float*)dev((size_t)F * cplane * 4);
+    if (c) {
+      cudaMemsetAsync(c, 0, (size_t)F * cplane * 4, st);
+      for (int f = 0; f < F; ++f)
+        cudaMemcpy2DAsync(c + f * cplane + 3 * ((size_t)r * Wp + pad_l), (size_t)Wp * 12, color + (size_t)f * h * w * 3, (size_t)w * 12, (size_t)w * 12, h, cudaMemcpyHostToDevice, st);
+    }
+    a.color = c;
+  }
+  a.out_frames = (const int*)up(out_frames, (size_t)q.num_out * 4);
+  a.retrans = (const int*)up(retrans.data(), retrans.size() * 4);
+  if (in_place) a.xparams = (const double*)up(xp.data(), xp.size() * 8);
+  a.out = (float*)dev((size_t)q.num_out * h * w * 4);
+  if (q.median) a.scratch = (float2*)dev((size_t)zmax * band * row_scratch);
+  int rc = RCVD_OK;
+  CUtensorMap tmd, tmc;
+  if (!ok) rc = set_err(RCVD_ERR_CUDA, "device allocation failed in rcvd_bilateral_filter");
+  else if (!encode_f32_3d(&tmd, a.depth, Wp, Hp, P, (uint64_t)Wp * 4, dplane * 4, box_w, box_h) ||
+           (use_c && !encode_f32_3d(&tmc, (void*)a.color, 3 * (uint64_t)Wp, Hp, F, (uint64_t)Wp * 12, cplane * 4, cbox_w, box_h)))
+    rc = set_err(RCVD_ERR_CUDA, "cuTensorMapEncodeTiled unavailable or failed: the TMA-fed bilateral filter cannot run");
+  else {
+    if (!use_c) tmc = tmd;   // not read
+    if (xform_cfg && in_place) a.cfg = *xform_cfg;
+    a.L = L; a.F = F; a.w = w; a.h = h; a.Wp = Wp; a.Hp = Hp; a.pad_l = pad_l;
+    a.spatial_radius = r; a.frame_radius = q.frame_radius; a.max_samples = max_samples;
+    a.box_w = box_w; a.box_h = box_h; a.stage_bytes = stage_bytes; a.depth_bytes = depth_bytes;
+    a.depth_sigma2 = q.depth_sigma > 0.f ? q.depth_sigma * q.depth_sigma : 0.f;   // sqr(sigma) in float (:184-185)
+    a.color_sigma2 = use_c ? q.color_sigma * q.color_sigma : 0.f;
+    e = q.median ? (in_place ? bilateral_prepare<true, true>(smem) : bilateral_prepare<true, false>(smem))
+                 : (in_place ? bilateral_prepare<false, true>(smem) : bilateral_prepare<false, false>(smem));
+    // in place: one launch per frame in range order; each reads the re-transformed planes written by the launches before it
+    for (int k0 = 0; e == cudaSuccess && k0 < q.num_out; k0 += zmax)
+      for (int y0 = 0; y0 < h; y0 += band) {
+        const int nz = std::min(zmax, q.num_out - k0), y1 = std::min(h, y0 + band);
+        a.out_begin = k0; a.y_begin = y0; a.y_end = y1;
+        const dim3 grid((w + kBilTW - 1) / kBilTW, (y1 - y0 + kBilTH - 1) / kBilTH, nz);
+        if (q.median) { if (in_place) bilateral_launch<true, true>(grid, smem, st, tmd, tmc, a); else bilateral_launch<true, false>(grid, smem, st, tmd, tmc, a); }
+        else { if (in_place) bilateral_launch<false, true>(grid, smem, st, tmd, tmc, a); else bilateral_launch<false, false>(grid, smem, st, tmd, tmc, a); }
+        g_filter_launches++;
+      }
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, a.out, (size_t)q.num_out * h * w * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) rc = set_err(RCVD_ERR_CUDA, "bilateral filter failed: %s", cudaGetErrorString(e));
+  }
+  for (void* b : bufs) cudaFreeAsync(b, st);
+  cudaStreamSynchronize(st); cudaStreamDestroy(st);
+  return rc;
+}
 
 // ---------------------------------------------------------------------------
 // GPU flow-constraint builder (rcvd_builder.cuh)

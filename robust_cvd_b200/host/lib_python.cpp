@@ -229,6 +229,7 @@ PYBIND11_MODULE(lib_python, m) {
   dvp.def(py::init<DepthVideo*>(), py::keep_alive<1, 2>())
       .def("process", &DepthVideoProcessor::process).def("gridXformSplit", &DepthVideoProcessor::gridXformSplit)
       .def("reset", &DepthVideoProcessor::reset).def("copy", &DepthVideoProcessor::copy).def("flowGuidedFilter", &DepthVideoProcessor::flowGuidedFilter)
+      .def("bilateralFilter", &DepthVideoProcessor::bilateralFilter)
       .def("resetPoses", &DepthVideoProcessor::resetPoses).def("resetDepthXforms", &DepthVideoProcessor::resetDepthXforms)
       .def("resetSpatialXforms", &DepthVideoProcessor::resetSpatialXforms)
       .def("normalizeDepth", &DepthVideoProcessor::normalizeDepth).def("optimizePoses", &DepthVideoProcessor::optimizePoses);

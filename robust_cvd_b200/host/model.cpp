@@ -254,7 +254,7 @@ std::string Xform::str() const {
   for (size_t i = 0; i < params_.size(); ++i) { snprintf(b, sizeof(b), "%s%.2f", i ? ", " : "", params_[i]); res += b; }
   return res + "]";
 }
-static void denseConfig(const XformDescriptor& d, rcvd_config& cfg) {
+void denseConfig(const XformDescriptor& d, rcvd_config& cfg) {
   memset(&cfg, 0, sizeof(cfg)); cfg.num_frames = 1; cfg.depth_type = RCVD_DEPTH_IDENTITY; cfg.value_xform = RCVD_VALUE_SCALE; cfg.spatial_type = RCVD_SPATIAL_IDENTITY;
   if (d.type == XformType::Depth) fillDepthConfig(d, cfg); else fillSpatialConfig(d, cfg);
   if (cfg.value_xform == RCVD_VALUE_NONE) cfg.value_xform = RCVD_VALUE_SCALE;

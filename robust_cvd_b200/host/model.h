@@ -146,6 +146,8 @@ class Xform {
 };
 void fillDepthConfig(const XformDescriptor& d, rcvd_config& cfg);
 void fillSpatialConfig(const XformDescriptor& d, rcvd_config& cfg);
+// the one-frame rcvd_config the dense kernels (rcvd_depth_apply, rcvd_depth_param_map, rcvd_spatial_warp) take for a transform
+void denseConfig(const XformDescriptor& d, rcvd_config& cfg);
 
 // --- DepthPhoto::Intrinsics / Extrinsics (lib/DepthPhoto.{h,cpp}) ---
 struct Extrinsics {
@@ -381,6 +383,7 @@ class DepthVideoProcessor {
   void process(const Params& params);
   void reset(const Params& params);               // lib/Processor.cpp:146-150
   void copy(const Params& params);                // :152-180
+  void bilateralFilter(const Params& params);     // :183-313, on the GPU (rcvd_bilateral_filter)
   void flowGuidedFilter(const Params& params);    // :315-590, on the GPU (rcvd_flow_guided_filter)
   void gridXformSplit(const Params& params);      // lib/Processor.cpp:888-985
   void resetPoses(const Params& params);          // :987-1003

@@ -310,8 +310,7 @@ void DepthVideoProcessor::process(const Params& params) {   // lib/Processor.cpp
     case Op::Reset: reset(params); break;
     case Op::Copy: copy(params); break;
     case Op::FlowGuidedFilter: flowGuidedFilter(params); break;
-    case Op::BilateralFilter:
-      throw std::runtime_error("The bilateral depth filter is outside the pose-optimization path and is not implemented in this build.");
+    case Op::BilateralFilter: bilateralFilter(params); break;
     default: throw std::runtime_error("Unsupported operation selected.");
   }
 }
@@ -331,6 +330,77 @@ void DepthVideoProcessor::copy(const Params& params) {   // :152-180
     dst.intrinsics = src.intrinsics; dst.extrinsics = src.extrinsics;
   }
 }
+// Bilateral filter (:183-313).  The reference filters frame by frame on the CPU, reading depth stream 0 and the "down" colour
+// stream whatever params.sourceDepthStream / colorStream say.  Here the host gathers the transformed depth of every frame a
+// temporal window reaches (and the colour only when the colour term is on) and rcvd_bilateral_filter (csrc/rcvd_bilateral.cuh)
+// filters the whole range.  With depthStream == 0 the reference's write-back between frames is honoured on the device: a later
+// window reads the depth transform applied to an earlier filtered frame, exactly what depth() returns after setDepth.
+void DepthVideoProcessor::bilateralFilter(const Params& params) {
+  logInfo("Applying bilateral filter...");
+  // every argument is checked before the first depth() call: depth() applies the transform on the GPU
+  if (params.spatialRadius < 0 || params.frameRadius < 0) throw std::runtime_error("Spatial and frame radius must be non-negative.");
+  params.frameRange.checkEmpty();
+  const int numFrames = video_->numFrames(), R = params.frameRadius;
+  const int first = params.frameRange.firstFrame(), last = params.frameRange.lastFrame();
+  if (first < 0 || last >= numFrames) throw std::runtime_error("Frame index out of range.");
+  DepthStream& ds = video_->depthStream(0);
+  DepthStream& dstDs = video_->depthStream(params.depthStream);
+  ColorStream& cs = video_->colorStream("down");
+  if (cs.type() != cvMakeType(CV_32F, 3)) throw std::runtime_error("Image has incorrect type.");   // ColorFrame::image3f
+  const bool useColor = params.colorSigma > 0.f, inPlace = params.depthStream == 0;
+  const int base = std::max(0, first - R), F = std::min(numFrames - 1, last + R) - base + 1;
+  std::vector<char> reached(F, 0);
+  for (int f : params.frameRange.frames) for (int g = std::max(0, f - R); g <= std::min(numFrames - 1, f + R); ++g) reached[g - base] = 1;
+  const int w = ds.width(), h = ds.height();
+  if (w <= 0 || h <= 0) throw std::runtime_error("Depth stream 0 has no depth frames.");
+  for (int i = 0; i < F; ++i) {
+    if (!reached[i]) continue;
+    if (!ds.frame(base + i).sourceDepth()) throw std::runtime_error("Depth frame " + std::to_string(base + i) + " has no depth image.");
+    if (useColor) {
+      const Image* c = cs.frame(base + i).image();
+      if (!c) throw std::runtime_error("Color frame " + std::to_string(base + i) + " has no image.");
+      if (c->cols != w || c->rows != h) throw std::runtime_error("Color frame " + std::to_string(base + i) + " does not have the depth frame's size.");
+    }
+  }
+  std::vector<int32_t> outFrames;
+  for (int f : params.frameRange.frames) outFrames.push_back(f - base);
+  // in place: the depth transform of every output frame, applied again to its filtered image on the device
+  rcvd_config cfg{}; std::vector<double> xp(1, 0.0);
+  const bool chain = inPlace && R > 0;
+  if (chain) {
+    const XformDescriptor& desc = ds.frame(first).depthXform().desc();
+    denseConfig(desc, cfg);
+    const int nd = rcvd_spatial_param_offset(&cfg) - rcvd_depth_param_offset(&cfg);
+    if (nd < 0) throw std::runtime_error("Unsupported depth transform for in-place filtering.");
+    xp.assign(std::max<size_t>(1, size_t(outFrames.size()) * nd), 0.0);
+    for (size_t k = 0; k < outFrames.size(); ++k) {
+      const Xform& x = ds.frame(base + outFrames[k]).depthXform();
+      if (x.desc() != desc || x.numParams() != nd) throw std::runtime_error("Depth transforms of the frame range differ.");
+      std::copy(x.params().begin(), x.params().end(), xp.begin() + k * nd);
+    }
+  }
+  std::vector<float> depth(size_t(F) * w * h, 0.f), color(useColor ? size_t(F) * w * h * 3 : 0);
+  for (int i = 0; i < F; ++i) {
+    if (!reached[i]) continue;
+    const Image* d = ds.frame(base + i).depth();
+    std::memcpy(depth.data() + size_t(i) * w * h, d->ptr<float>(), size_t(w) * h * sizeof(float));
+    if (useColor) std::memcpy(color.data() + size_t(i) * w * h * 3, cs.frame(base + i).image()->ptr<float>(), size_t(w) * h * 3 * sizeof(float));
+  }
+  rcvd_bilateral_params prm{};
+  prm.num_frames = F; prm.num_out = int(outFrames.size()); prm.width = w; prm.height = h;
+  prm.spatial_radius = params.spatialRadius; prm.frame_radius = R; prm.median = params.median ? 1 : 0; prm.in_place = inPlace ? 1 : 0;
+  prm.depth_sigma = params.depthSigma; prm.color_sigma = params.colorSigma;
+  std::vector<float> out(size_t(prm.num_out) * w * h);
+  const int rc = rcvd_bilateral_filter(&prm, currentDevice(), depth.data(), useColor ? color.data() : nullptr, outFrames.data(),
+                                       chain ? &cfg : nullptr, chain ? xp.data() : nullptr, out.data());
+  if (rc != RCVD_OK) throw std::runtime_error(std::string("bilateral filter failed: ") + rcvd_last_error());
+  for (size_t k = 0; k < outFrames.size(); ++k) {   // range order, as the reference writes
+    Image img; img.create(h, w, cvMakeType(CV_32F, 1));
+    std::memcpy(img.ptr<float>(), out.data() + k * w * h, size_t(w) * h * sizeof(float));
+    dstDs.frame(base + outFrames[k]).setDepth(img);
+  }
+}
+
 // Flow-guided temporal filter (:315-590).  The reference walks frame by frame and pixel by pixel on the CPU; here the host
 // gathers the depth images, cameras and consecutive-frame flows of the whole range once and one kernel launch
 // (rcvd_flow_guided_filter, csrc/rcvd_filter.cuh) filters every frame.

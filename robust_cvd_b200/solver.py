@@ -277,6 +277,26 @@ def flow_guided_filter(depth, cams, fwd_flow, fwd_mask, bwd_flow, bwd_mask, firs
     return out
 
 
+def bilateral_filter(depth, out_frames, frame_radius=2, spatial_radius=0, depth_sigma=0.3, color_sigma=0.0, median=False, color=None,
+                     in_place=False, xform_cfg=None, xform_params=None, device=0):
+    """rcvd_bilateral_filter (DepthVideoProcessor::bilateralFilter, reference lib/Processor.cpp:183-313) on the GPU.
+    depth [F,h,w] f32 (transformed depth of stream 0), color [F,h,w,3] f32 or None, out_frames ascending frame indices
+    -> filtered depth [len(out_frames),h,w] f32.  in_place: each filtered frame replaces its depth, with the transform
+    (xform_cfg, xform_params [len(out_frames), depth params]) applied again, before later windows read it."""
+    depth = np.ascontiguousarray(depth, np.float32); F, h, w = depth.shape
+    col = None if color is None else np.ascontiguousarray(color, np.float32)
+    of = np.ascontiguousarray(out_frames, np.int32).reshape(-1)
+    xp = None if xform_params is None else np.ascontiguousarray(xform_params, np.float64)
+    if xp is not None and xp.size == 0:
+        xp = np.zeros(1, np.float64)        # a transform without parameters (identity)
+    prm = abi.BilateralParams(num_frames=F, num_out=len(of), width=w, height=h, spatial_radius=spatial_radius, frame_radius=frame_radius,
+                              median=1 if median else 0, in_place=1 if in_place else 0, depth_sigma=depth_sigma, color_sigma=color_sigma)
+    out = np.zeros((len(of), h, w), np.float32)
+    _check(lib().rcvd_bilateral_filter(C.byref(prm), C.c_int32(device), _p(depth, C.c_float), _p(col, C.c_float), _p(of, C.c_int32),
+                                       C.byref(xform_cfg) if xform_cfg is not None else None, _p(xp, C.c_double), _p(out, C.c_float)))
+    return out
+
+
 def build_constraints(color_bgr, pair_frames, pair_flow, pair_mask, match_separation, inv_aspect, dyn_dist=None, min_dynamic_distance=-1.0,
                       trip_frames=None, trip_flow=None, trip_mask=None, device=0):
     """rcvd_build_constraints (FlowConstraintsCollection::compute + sampleConstraints, reference lib/FlowConstraints.cpp:352-550) on the GPU.
